@@ -273,8 +273,17 @@ def gpu_baseline(scene, w, h, calls=6):
             "note": "a different, fast-math estimator (SURVEY 2 row 3): speed bar only, not a parity arm"}
 
 
-def measure_one_gpu(tb, torch, np, scene, w, h, spp, steps, warmup, device, flush, want_clocks=False):
-    """Single-GPU measurement of one configuration: device-resident value + e2e through tb200_render."""
+def dump_outputs(np, outdir, accum):
+    """Writes what the timed path hands its caller after the last timed step: the accumulator, (H, W, 4)
+    float32 running sums (sum w*rgb, sum w) over every timed sample.  r.Init resets the frame index, so
+    the same --steps give the same samples whatever --warmup is."""
+    os.makedirs(outdir, exist_ok=True)
+    np.save(os.path.join(outdir, "accumulator.npy"), np.ascontiguousarray(accum, np.float32))
+
+
+def measure_one_gpu(tb, torch, np, scene, w, h, spp, steps, warmup, device, flush, want_clocks=False, dump=None):
+    """Single-GPU measurement of one configuration: device-resident value + e2e through tb200_render.
+    dump: directory for the timed path's output (dump_outputs)."""
     snap = tb.Snapshot(tb.scene_path(scene))
     cam, opt = snap.camera, snap.options
     opt.width, opt.height = w, h
@@ -311,6 +320,8 @@ def measure_one_gpu(tb, torch, np, scene, w, h, spp, steps, warmup, device, flus
         step_ms = lib_ms
         launches = r.stats().kernelLaunches - launches0
         img = r.read_accumulator()
+    if dump:
+        dump_outputs(np, dump, img)
     value = w * h * spp * steps / sum(step_ms) / 1e3
 
     # sanity: filter weights sum to spp per interior pixel
@@ -361,7 +372,8 @@ def run_ours(args):
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
 
     if world == 1:
-        res = measure_one_gpu(tb, torch, np, scene, W, H, SPP, args.steps, args.warmup, local, flush, want_clocks=True)
+        res = measure_one_gpu(tb, torch, np, scene, W, H, SPP, args.steps, args.warmup, local, flush, want_clocks=True,
+                              dump=args.dump_outputs)
         value, step_ms = res["value"], res["step_ms"]
         avg_launch_s = sum(step_ms) / len(step_ms) / 1e3
         line = {
@@ -487,6 +499,8 @@ def run_ours(args):
     if rank == 0:
         img = accum.cpu().numpy()
         assert np.isfinite(img).all() and float(img[..., :3].sum()) > 0.0
+        if args.dump_outputs:
+            dump_outputs(np, args.dump_outputs, img)
     r.close()
     del accum
     torch.cuda.synchronize()
@@ -555,7 +569,12 @@ def main():
     ap.add_argument("--scene", default="cornell", choices=["cornell"] + sorted(OTHER_WORKLOADS),
                     help="run another BASELINE.json configuration as the main workload (development)")
     ap.add_argument("--no-configs", action="store_true", help="skip the sub-results for the other BASELINE.json configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed path's output after the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's output: use it with --impl ours")
     if args.scene != "cornell":
         global MAIN
         w, h, spp = OTHER_WORKLOADS[args.scene]

@@ -30,6 +30,18 @@
 #include "tb200_detmath.h"
 #include "tinsel_b200.h"
 
+// -DTB_ORACLE_LIBM (libtinsel_oracle_libm.so): the transcendentals come from the system libm, as in the
+// reference as shipped (the "literal" flavour of oracle/_ref); the default build uses the deterministic
+// ones the kernels use, so only this flavour may differ from the CUDA path, in the last bits.
+#ifdef TB_ORACLE_LIBM
+#define tbm_sinf sinf
+#define tbm_cosf cosf
+#define tbm_expf expf
+#define tbm_powf powf
+#define tbm_acosf acosf
+#define tbm_atan2f atan2f
+#endif
+
 // Optional work counters (-DTB_ORACLE_COUNT, built as libtinsel_oracle_count.so): the inputs of the
 // ALGORITHMIC-bytes formula of SURVEY.md 8(d), counted on the reference traversal order.
 enum { C_VINT, C_TTRI, C_TPRIM, C_HMESH, C_HIT, C_NEE_BYTES, C_PROBE_BYTES, C_MISS_BYTES, C_FB_PIXELS, C_RAYS, C_SAMPLES, C_NUM };

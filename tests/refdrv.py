@@ -212,19 +212,22 @@ class RefScene:
 
 # ---- the CPU restatement (oracle/libtinsel_oracle.so) ---------------------------------------------
 
-PORT_PATH = os.path.join(ROOT, "oracle", "libtinsel_oracle.so")
-_port = None
+# "detmath": the deterministic transcendentals the kernels use; "literal": the system libm's, as the
+# reference ships (oracle/Makefile port)
+PORT_PATHS = {"detmath": os.path.join(ROOT, "oracle", "libtinsel_oracle.so"),
+              "literal": os.path.join(ROOT, "oracle", "libtinsel_oracle_libm.so")}
+PORT_PATH = PORT_PATHS["detmath"]
+_ports = {}
 
 
 def have_port():
     return os.path.exists(PORT_PATH)
 
 
-def load_port():
-    global _port
-    if _port is not None:
-        return _port
-    lib = C.CDLL(PORT_PATH)
+def load_port(flavour="detmath"):
+    if flavour in _ports:
+        return _ports[flavour]
+    lib = C.CDLL(PORT_PATHS[flavour])
     lib.oracle_create.restype = C.c_void_p
     lib.oracle_create.argtypes = [C.POINTER(abi.Scene)]
     lib.oracle_destroy.argtypes = [C.c_void_p]
@@ -250,31 +253,35 @@ def load_port():
     lib.oracle_quantize.argtypes = [_f32p, C.c_int, C.POINTER(C.c_ubyte)]
     lib.oracle_nlm.argtypes = [_f32p, _f32p, C.c_int, C.c_int, C.c_float, C.c_int]
     abi.declare_snapshot_api(lib)
-    _port = lib
+    _ports[flavour] = lib
     return lib
 
 
 class PortScene:
     """The CPU restatement over a tb200_scene (from a snapshot or any tb200_scene view)."""
 
-    def __init__(self, scene_ptr, camera, options, keepalive=None):
-        self.lib = load_port()
+    def __init__(self, scene_ptr, camera, options, keepalive=None, flavour="detmath"):
+        self.lib = load_port(flavour)
         self.h = C.c_void_p(self.lib.oracle_create(scene_ptr))
         self.camera = abi.copy_struct(camera)
         self.options = abi.copy_struct(options)
         self._keep = keepalive
 
     @classmethod
-    def from_snapshot(cls, path):
-        lib = load_port()
+    def from_snapshot(cls, path, flavour="detmath"):
+        lib = load_port(flavour)
         h = lib.tb200_snapshot_load(path.encode())
         if not h:
             raise RuntimeError("cannot load " + path)
         scene = lib.tb200_snapshot_scene(h)
-        return cls(scene, lib.tb200_snapshot_camera(h).contents, lib.tb200_snapshot_options(h).contents, keepalive=h)
+        return cls(scene, lib.tb200_snapshot_camera(h).contents, lib.tb200_snapshot_options(h).contents, keepalive=h,
+                   flavour=flavour)
 
     def set_size(self, w, h):
         self.options.width, self.options.height = w, h
+
+    def set_max_depth(self, d):
+        self.options.maxDepth = d
 
     def render_seeded(self, frame0, nframes, nthreads=1, out=None):
         o = self.options
@@ -282,6 +289,8 @@ class PortScene:
             out = np.zeros((o.height, o.width, 4), np.float32)
         self.lib.oracle_render_seeded(self.h, C.byref(self.camera), C.byref(o), frame0, nframes, _fp(out), nthreads)
         return out
+
+    render_pool = render_seeded   # RefScene.render_pool computes the same samples, only scheduled differently
 
     def trace_frame(self, frame, nthreads=1):
         o = self.options

@@ -17,6 +17,7 @@ import pytest
 import tinsel_b200 as tb
 from tinsel_b200 import abi
 import refdrv
+import genscenes
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -95,12 +96,13 @@ def _biggest_mesh(scene):
     return best
 
 
-@pytest.mark.parametrize("name,size", [("glass", (128, 128)), ("meshlight", (128, 128)), ("table", (160, 100)), ("ajax", (192, 192))])
+@pytest.mark.parametrize("name,size", [("glass", (128, 128)), ("meshlight", (128, 128)), ("table", (160, 100)), ("ajax", (192, 192)),
+                                       ("instances", (160, 100)), ("bigmesh", (192, 192))])
 def test_gpu_built_bvh_structure_and_parity(name, size):
-    if not os.path.exists(tb.scene_path(name)):
+    if not os.path.exists(genscenes.path(name)):
         pytest.skip("snapshot scenes/%s.tsnap not present" % name)
     os.environ["TINSEL_B200_PIPELINE"] = "wavefront"
-    snap = tb.Snapshot(tb.scene_path(name))
+    snap = tb.Snapshot(genscenes.path(name))
     cam, opt = snap.camera, snap.options
     opt.width, opt.height = size
     m = _biggest_mesh(snap.scene.contents)

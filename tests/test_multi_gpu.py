@@ -11,6 +11,7 @@ import pytest
 import tinsel_b200 as tb
 from tinsel_b200 import abi, sharding
 import refdrv
+import genscenes
 
 pytestmark = pytest.mark.gpu
 
@@ -21,10 +22,10 @@ def _gpus():
 
 
 def _scene(name, size):
-    if not os.path.exists(tb.scene_path(name)):
+    if not os.path.exists(genscenes.path(name)):
         pytest.skip("snapshot scenes/%s.tsnap not present" % name)
     os.environ["TINSEL_B200_PIPELINE"] = "wavefront"
-    snap = tb.Snapshot(tb.scene_path(name))
+    snap = tb.Snapshot(genscenes.path(name))
     cam, opt = snap.camera, snap.options
     opt.width, opt.height = size
     return snap, cam, opt
@@ -41,7 +42,7 @@ def _single(snap, cam, opt, spp):
 
 
 @pytest.mark.parametrize("name,size,parts", [("cornell", (200, 150), 3), ("veach", (160, 90), 2), ("cornell", (64, 9), 4),
-                                             ("ajax", (96, 96), 3)])
+                                             ("ajax", (96, 96), 3), ("bigmesh", (96, 96), 3)])
 def test_row_slabs_compose_the_image_on_one_device(name, size, parts):
     """tb200_set_slab: `parts` renderers, each owning one slab, all Render() into the SAME host buffer;
     every row is written by its owner only, and the composed image is the unsharded one (same

@@ -9,6 +9,7 @@ import pytest
 import tinsel_b200 as tb
 from tinsel_b200 import abi
 import refdrv
+import genscenes
 
 pytestmark = pytest.mark.gpu
 
@@ -30,24 +31,33 @@ SCENES = {
     "table": (160, 100),   # 15 primitives, 5 meshes (prisms, cubes, quads) on a table: glass, metal, many instances
     "simple": (96, 48),    # two primitives
     "envmini": (128, 96),  # HDR-probe lighting only (synthetic 128x64 probe): ProbeSample / ProbePdf / ProbeEval
+    # generated from a seed (tests/genscenes.py), standing in for ajax, env and table where those are absent
+    "bigmesh": (160, 160),
+    "bigenv": (160, 160),
+    "instances": (160, 100),
 }
 
 
 def _available(name):
-    return os.path.exists(tb.scene_path(name))
+    return os.path.exists(genscenes.path(name))
 
 
 def _setup(name, pipeline, size=None, flavour="detmath"):
+    """The oracle is the reference's own code when oracle/_ref is built, and otherwise the CPU restatement
+    (oracle/tinsel_oracle.cpp), which test_oracle.py pins bit for bit to the reference's outputs stored in
+    tests/golden; for the literal flavour the restatement is built with the system libm, as the reference ships."""
     if not _available(name):
         pytest.skip("snapshot scenes/%s.tsnap not present" % name)
-    if not refdrv.have_ref(flavour):
-        pytest.skip("oracle/_ref not built")
     os.environ["TINSEL_B200_PIPELINE"] = pipeline
-    snap = tb.Snapshot(tb.scene_path(name))
+    path = genscenes.path(name)
+    snap = tb.Snapshot(path)
     cam, opt = snap.camera, snap.options
     w, h = size or SCENES[name]
     opt.width, opt.height = w, h
-    ref = refdrv.RefScene.from_snapshot(tb.scene_path(name), flavour=flavour)
+    if refdrv.have_ref(flavour):
+        ref = refdrv.RefScene.from_snapshot(path, flavour=flavour)
+    else:
+        ref = refdrv.PortScene.from_snapshot(path, flavour=flavour)
     ref.set_size(w, h)
     r = tb.Renderer(snap.scene)
     r.Init(w, h)
@@ -79,7 +89,7 @@ def test_per_sample_radiance_bit_exact(name, pipeline):
 
 
 @pytest.mark.parametrize("pipeline", ["mega", "wavefront"])
-@pytest.mark.parametrize("name", ["cornell", "veach", "glass", "ajax", "env", "envmini"])
+@pytest.mark.parametrize("name", ["cornell", "veach", "glass", "ajax", "env", "envmini", "bigmesh", "bigenv"])
 def test_render_matches_seeded_oracle(name, pipeline):
     """Renderer.Render x spp vs oracle B at matched spp and seeds: rel-L2 <= 1e-4 (BASELINE.json)."""
     snap, cam, opt, ref, r = _setup(name, pipeline)
@@ -99,15 +109,20 @@ def test_render_matches_seeded_oracle(name, pipeline):
     snap.close()
 
 
-@pytest.mark.parametrize("name", ["cornell", "veach", "meshlight", "ajax"])
+@pytest.mark.parametrize("name", ["cornell", "veach", "meshlight", "ajax", "bigmesh"])
 def test_normals_mode_bit_exact_vs_literal_reference(name):
-    """eNormals (render.cpp:494-515) has no RNG and no libm: exact match against the literal reference."""
+    """eNormals (render.cpp:494-515) has no RNG and no libm: exact match against the literal reference, or
+    without oracle/_ref against the CPU restatement's normals image (pinned to the reference's in tests/golden)."""
+    literal = refdrv.have_ref("literal")
     snap, cam, opt, ref, r = _setup(name, "wavefront", flavour="literal")
     opt.mode = abi.MODE_NORMALS
-    ref.set_mode(abi.MODE_NORMALS)
     out = np.zeros((opt.height, opt.width, 4), np.float32)
     r.Render(cam, opt, out)
-    expect = ref.render_literal(1)
+    if literal:
+        ref.set_mode(abi.MODE_NORMALS)
+        expect = ref.render_literal(1)
+    else:
+        expect = ref.render_normals()
     assert np.array_equal(out.view(np.uint32), expect.view(np.uint32)), \
         "%d pixels differ" % int((out != expect).any(-1).sum())
     r.close()
@@ -232,7 +247,7 @@ def test_both_scheduling_modes_bit_exact(sched, cta):
         os.environ["TINSEL_B200_WALKERS"] = sched[len("offload"):]
     os.environ["TINSEL_B200_CTA"] = cta
     try:
-        for name in ("veach", "meshlight", "many", "envmini", "glass", "table", "ajax", "motionblur"):
+        for name in ("veach", "meshlight", "many", "envmini", "glass", "table", "ajax", "motionblur", "bigmesh", "instances"):
             if not _available(name):
                 continue
             snap, cam, opt, ref, r = _setup(name, "wavefront")
@@ -351,9 +366,10 @@ def test_lane_queue_layout_on_small_frames(monkeypatch):
 # BASELINE.json configs at their full image sizes (C2 cornell 1024^2, C3 ajax 1024^2, C4 veach
 # 1920x1080 with clamp 4, C5 env 2048^2): one frame of every config traced per sample on the GPU
 # and by the reference's PathTrace on all host cores -- bit-exact -- and the same frame through
-# Render() against the seeded oracle image.
+# Render() against the seeded oracle image.  bigmesh and bigenv (tests/genscenes.py) take ajax's and env's
+# roles at 1024^2 where those snapshots are absent.
 @pytest.mark.parametrize("name,size", [("cornell", (1024, 1024)), ("ajax", (1024, 1024)), ("veach", (1920, 1080)),
-                                       ("env", (2048, 2048))])
+                                       ("env", (2048, 2048)), ("bigmesh", (1024, 1024)), ("bigenv", (1024, 1024))])
 def test_baseline_configs_full_size(name, size):
     snap, cam, opt, ref, r = _setup(name, "wavefront", size=size)
     threads = min(os.cpu_count() or 8, 32)   # the box runs under a 16-CPU cgroup quota: more threads only thrash
@@ -393,7 +409,8 @@ LITERAL_REPORT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__
 # Its bound is therefore on the pixels: all but a 1e-4 fraction of them agree to 1e-3, and the image to 5e-3.
 @pytest.mark.parametrize("name,size,spp,tol", [("cornell", (1024, 1024), 8, 1e-4), ("ajax", (1024, 1024), 8, 1e-4),
                                                ("veach", (1920, 1080), 8, 1e-4), ("env", (2048, 2048), 32, 1e-4),
-                                               ("glass", (512, 512), 8, 5e-3)])
+                                               ("glass", (512, 512), 8, 5e-3), ("bigmesh", (1024, 1024), 8, 1e-4),
+                                               ("bigenv", (1024, 1024), 32, 1e-4)])
 def test_literal_reference_rel_l2_at_baseline_sizes(name, size, spp, tol):
     snap, cam, opt, ref, r = _setup(name, "wavefront", size=size, flavour="literal")
     threads = min(os.cpu_count() or 8, 32)

@@ -9,12 +9,13 @@ import numpy as np
 import pytest
 
 import tinsel_b200 as tb
+import genscenes
 
 
 def _cache(tmp_path, name):
-    if not os.path.exists(tb.scene_path(name)):
+    if not os.path.exists(genscenes.path(name)):
         pytest.skip("snapshot scenes/%s.tsnap not present" % name)
-    snap = tb.Snapshot(tb.scene_path(name))
+    snap = tb.Snapshot(genscenes.path(name))
     path = str(tmp_path / (name + ".tcache"))
     tb.scene_cache_save(snap.scene, path)
     return snap, path
@@ -73,7 +74,7 @@ def test_damaged_cache_files_are_refused(tmp_path):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name,size", [("glass", (128, 128)), ("envmini", (128, 96)), ("ajax", (160, 160)), ("veach", (192, 108)),
-                                       ("env", (256, 256))])
+                                       ("env", (256, 256)), ("bigmesh", (160, 160)), ("bigenv", (256, 256))])
 def test_renderer_from_cache_is_bit_identical(tmp_path, name, size):
     snap, path = _cache(tmp_path, name)
     os.environ["TINSEL_B200_PIPELINE"] = "wavefront"
